@@ -15,6 +15,10 @@ GPU (BASELINE.json configs[1]; weak scaling, so N GPUs = configs[4]'s 256/GPU).
   roofline  the dominant kernel's algorithmic bytes / its CUDA-event time (DESIGN.md)
   cpu_baseline  the reference itself (oracle/_ref, parallelMap on all host threads) on a
           bounded sample of the same workload
+
+Every timed region runs exactly --steps steps after --warmup untimed ones.  --dump-outputs DIR writes what
+the device leg returned in its last timed step (see dump_outputs), so that two builds can be compared output
+for output: the inputs are seeded, identical from run to run for the same arguments.
 """
 import argparse
 import json
@@ -40,6 +44,24 @@ def make_inputs(first, count, T, C, U):
         e[i] = rng.uniform(-5.0, 5.0, (T, C)).astype(np.float32)
         tg.append(rng.integers(1, C, U).astype(np.int32))
     return e, tg
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, outputs):
+    """outputs: {name: array whose first axis is the utterance}, written as path/<name>.npy in float32 or
+    float64 (integer outputs as float64, which holds them exactly).  When they exceed DUMP_BYTES together,
+    every array keeps the same utterances: a sorted sample drawn with a fixed seed, as many as fit."""
+    os.makedirs(path, exist_ok=True)
+    outputs = {k: (v.astype(np.float64) if v.dtype.kind in "iu" else v) for k, v in outputs.items()}
+    B = len(next(iter(outputs.values())))
+    per_utt = sum(v.nbytes for v in outputs.values()) // B
+    keep = np.arange(B)
+    if per_utt * B > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(B, DUMP_BYTES // per_utt, replace=False))
+    for k, v in outputs.items():
+        np.save(os.path.join(path, k + ".npy"), np.ascontiguousarray(v[keep]))
 
 
 def ctc_view(capi, target, blank=0):
@@ -206,7 +228,7 @@ def cpu_reference(sample, T, C, U, repeats=1, keep=None):
                       % (sample, T, C, U, min(cores, sample)), "seconds": best}
 
 
-def api_path_leg(e, tg, T, C, steps=5):
+def api_path_leg(e, tg, T, C, steps):
     """The drop-in path a user gets by swapping the import: the reference's Python surface (gtn_b200.gtn), one
     Graph per utterance, the LIST forms of intersect / forward_score / subtract / backward (bindings/python/
     gtn/_functions.cpp:69-135), emissions handed over as device pointers of a torch CUDA tensor
@@ -359,13 +381,13 @@ def run_other_workload(args, rank, local, world):
         n = min(args.cpu_sample, 16 if asg else 8)
         e, tg = inputs(0, n)
         step = (lambda: po.ref_asg_batch(e, tw, tg)[3]) if asg else (lambda: po.ref_viterbi_dense_batch(e, tw)[2])
-        for _ in range(min(args.warmup, 1)):
+        for _ in range(args.warmup):
             step()
-        secs = [step() for _ in range(max(1, min(args.steps, 3)))]
+        secs = [step() for _ in range(args.steps)]
         val = n / float(np.mean(secs))
         print(json.dumps({
             "impl": "reference", "metric": metric, "value": val, "unit": "utt/s", "n_gpus": args.gpus,
-            "steps": len(secs), "warmup": min(args.warmup, 1), "ms_per_step": 1e3 * float(np.mean(secs)),
+            "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * float(np.mean(secs)),
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": name, "parallelism": "dp%d" % world},
             "cpu_baseline": {"value": val, "unit": "utt/s", "cores": min(po.libref().ref_hardware_threads(), n),
@@ -458,6 +480,11 @@ def run_other_workload(args, rank, local, world):
     ts, pr, launches = region(step_dev, True)
     gpu_losses = losses.copy() if asg else scores.copy()
     gpu_paths = None if asg else paths.copy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"losses": gpu_losses, "grads": g_dev.download((B, T, C))} if asg else
+                     {"scores": gpu_losses, "paths": gpu_paths})
+        if asg:
+            np.save(os.path.join(args.dump_outputs, "transition_grads.npy"), tgrad)
     for _ in range(2):
         step_e2e()
     te, _, _ = region(step_e2e, False)
@@ -530,6 +557,9 @@ def main():
                     help="ctc only: --batch is the WHOLE job (configs[4]: B=2048 fixed), split over the ranks")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-api-path", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of the device leg as DIR/<name>.npy (rank 0's; "
+                         "at most 64 MB: above that, the same seeded sample of utterances of every output)")
     args = ap.parse_args()
     if args.batch is None:
         args.batch = 2048 if args.strong else B_DEF
@@ -663,39 +693,14 @@ def main():
             ctx.profile(False)
         return {"times": ts, "wall": w, "launches": ctx.launches - l0, "prof": pr}
 
-    def measure(step, profile):
-        """The GPU boxes are shared hosts: now and then a run is hit by multi-millisecond stalls
-        that are not ours (same binary: 0.55 ms steady in one process; in the next, single steps of
-        12 - 130 ms).  A region whose mean is more than 15 % above its own median is measured again,
-        at most twice, FOR INFORMATION: the first attempt is the one reported (no selection), every
-        attempt is listed in attempts_ms_per_step."""
-        tries = []
-        for _ in range(3):
-            r = timed_region(step, profile)
-            tries.append(r)
-            disturbed = float(np.mean(r["times"]) > 1.15 * np.median(r["times"]))
-            if world > 1:  # every rank takes the same decision (the region contains barriers)
-                f = torch.tensor([disturbed], device="cuda")
-                dist.all_reduce(f, op=dist.ReduceOp.MAX)
-                disturbed = float(f[0])
-            if not disturbed:
-                break
-        means = [float(np.mean(r["times"])) for r in tries]
-        if world > 1:  # an attempt counts with its slowest rank
-            m = torch.tensor(means, device="cuda", dtype=torch.float64)
-            dist.all_reduce(m, op=dist.ReduceOp.MAX)
-            means = [float(x) for x in m]
-        # the FIRST attempt is the reported one; later attempts are listed for information only
-        return tries[0], means
-
-    dev, dev_attempts = measure(step_dev, True)
+    dev = timed_region(step_dev, True)
     times, wall, launches, prof = dev["times"], dev["wall"], dev["launches"], dev["prof"]
     losses_dev_leg = losses.copy()  # the last timed step's losses; its gradients are still in g_dev
 
     # end-to-end leg (host buffers)
     for _ in range(2):
         step_e2e()
-    e2e, e2e_attempts = measure(step_e2e, False)
+    e2e = timed_region(step_e2e, False)
     e2e_times = e2e["times"]
     clocks = sampler.result()
 
@@ -750,10 +755,6 @@ def main():
             "numa": numa,
             "clocks": clocks,
             "ms_per_step_median": float(np.median(times)), "ms_per_step_min": float(np.min(times)),
-            "attempts_ms_per_step": {"value": dev_attempts, "e2e": e2e_attempts,
-                                     "policy": "the FIRST timed region is the one reported; a region whose mean exceeds 1.15 x "
-                                               "its median (stalls of the shared host) is measured again, at most twice, "
-                                               "and listed here for information"},
             "roofline": roofline,
             "roofline_whole_step_csr": {"achieved": b_csr / (ms * 1e-3) / 1e9, "unit": "GB/s",
                                         "frac": b_csr / (ms * 1e-3) / 1e9 / peak, "bytes": b_csr},
@@ -767,12 +768,14 @@ def main():
                 out["parity"] = parity_block(ctx, keep, losses_dev_leg, g_dev, T, C)
         if not args.no_api_path and world == 1:
             try:
-                api, al, ag = api_path_leg(e, tg, T, C)
+                api, al, ag = api_path_leg(e, tg, T, C, args.steps)
                 api["max_rel_loss_vs_fused"] = float((np.abs(al - losses_dev_leg) / np.abs(losses_dev_leg)).max())
                 api["max_abs_grad_vs_fused"] = float(np.abs(np.stack(ag[:16]).reshape(16, T, C) - g_dev.download((16, T, C))).max())
                 out["api_path"] = api
             except Exception as ex:  # the line must still print
                 out["api_path"] = {"error": str(ex)[:200]}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"losses": losses_dev_leg, "grads": g_dev.download((B, T, C))})
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()

@@ -1,14 +1,14 @@
 """k_gcompose.cu (general device composition: epsilons, cycles, any sortedness) run on the CPU through the SIMT
-emulator, against the live reference (oracle/_ref: detail::compose, compose.cpp:377-522): identical node
-numbering, arc numbering, labels, weights and gradInfo -- not merely isomorphic graphs."""
+emulator, against the reference (detail::compose, compose.cpp:377-522, its results on these seeded operands stored in
+tests/golden/reference_host.json): identical node numbering, arc numbering, labels, weights and gradInfo -- not merely
+isomorphic graphs."""
 import ctypes as C
 
 import numpy as np
 import pytest
 
-from oracle import pyoracle as po
-from tests import emu_build
-from tests.test_host_api import ours_arrays, ours_from, random_graph, ref_from
+from tests import emu_build, util
+from tests.test_host_api import golden, ours_arrays, ours_from, random_graph
 
 i32p, f32p, u8p = C.POINTER(C.c_int32), C.POINTER(C.c_float), C.POINTER(C.c_uint8)
 
@@ -98,30 +98,23 @@ def test_kernel_source_reproduces_the_reference_numbering(emu, gtn, seed):
         mb.arc_sort(False)
     # every third case: the co-reachability search on 2 or 3 concurrent CTAs (gcompose_reach_kernel)
     out = run(emu, gtn, ma, mb, intersect, reach_ctas=(1, 1, 2, 1, 1, 3)[seed % 6])
-    # the host construction of the gtn:: layer (pinned against the live reference by tests/test_host_api.py)
+    # the host construction of the gtn:: layer (pinned against the reference by tests/test_host_api.py)
     gtn.set_compose_device_policy(2)
     try:
         host = gtn.intersect(ma, mb) if intersect else gtn.compose(ma, mb)
     finally:
         gtn.set_compose_device_policy(0)
     check_against(out, ours_arrays(host), "vs the host construction")
-    if po.have_ref():
-        ta, tb = ref_from(a), ref_from(b)
-        if seed & 1:
-            ta.arc_sort(True)
-        if seed & 2:
-            tb.arc_sort(False)
-        to = po.ref_op("intersect" if intersect else "compose", ta, tb)
-        check_against(out, to.arrays(), "vs the reference")
-        # gradInfo (compose.cpp:445, 201-205): the scatter of random deltas equals the reference's backward
-        if len(out["src"]):
-            d = rng.integers(-5, 6, len(out["src"])).astype(np.float32)
-            seed_t = ref_from((out["flags"], out["src"], out["dst"], out["ilabel"], out["olabel"], d), calc_grad=False)
-            po.ref_backward_with(to, seed_t)
-            for gi, t, n in ((out["gi1"], ta, len(a[1])), (out["gi2"], tb, len(b[1]))):
-                g = np.zeros(n, np.float32)
-                np.add.at(g, gi[gi >= 0], d[gi >= 0])
-                assert np.array_equal(g, t.grad().weights())
+    want = golden("compose", seed)
+    check_against(out, util.graph_arrays(want["out"]), "vs the reference")
+    # gradInfo (compose.cpp:445, 201-205): the scatter of random deltas equals the reference's backward
+    assert (want["grads"] is not None) == bool(len(out["src"]))
+    if len(out["src"]):
+        d = rng.integers(-5, 6, len(out["src"])).astype(np.float32)
+        for gi, wg, n in ((out["gi1"], want["grads"][0], len(a[1])), (out["gi2"], want["grads"][1], len(b[1]))):
+            g = np.zeros(n, np.float32)
+            np.add.at(g, gi[gi >= 0], d[gi >= 0])
+            assert np.array_equal(g, np.array(wg, np.float32))
 
 
 @pytest.mark.parametrize("seed", range(4))

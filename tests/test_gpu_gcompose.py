@@ -1,12 +1,13 @@
 """General composition on the GPU (k_gcompose.cu through gtnb_compose_graphs and the gtn:: surface): arbitrary
-operand pairs -- epsilons, cycles, any sortedness -- against the live reference (oracle/_ref) where it was
-built, else against the host construction: identical numbering, weights and gradients."""
+operand pairs -- epsilons, cycles, any sortedness -- against the reference (its results on these seeded operands
+stored in tests/golden/reference_host.json) and against the host construction: identical numbering, weights and
+gradients."""
 import numpy as np
 import pytest
 
-from oracle import pyoracle as po
+from tests import util
 from tests.test_gcompose_emulation import case, check_against
-from tests.test_host_api import ours_arrays, ours_from, ref_from, seed_like
+from tests.test_host_api import golden, ours_arrays, ours_from, seed_like
 
 pytestmark = pytest.mark.gpu
 
@@ -51,20 +52,13 @@ def test_device_compose_matches_reference_numbering_and_gradients(gtn, on_device
         hb.arc_sort(False)
     ho = host(gtn, gtn.intersect if intersect else gtn.compose, ha, hb)
     check_against(ours_arrays(mo), ours_arrays(ho), "device vs host construction")
-    if po.have_ref():
-        ta, tb = ref_from(a), ref_from(b)
-        if seed & 1:
-            ta.arc_sort(True)
-        if seed & 2:
-            tb.arc_sort(False)
-        to = po.ref_op("intersect" if intersect else "compose", ta, tb)
-        check_against(ours_arrays(mo), to.arrays(), "device vs reference")
-        if mo.num_arcs():
-            seed_m, seed_t = seed_like(gtn, mo, rng)
-            gtn.backward(mo, seed_m)
-            po.ref_backward_with(to, seed_t)
-            for m, t in ((ma, ta), (mb, tb)):
-                assert np.array_equal(np.array(m.grad().weights_to_list(), np.float32).reshape(-1), t.grad().weights())
+    want = golden("compose", seed)
+    check_against(ours_arrays(mo), util.graph_arrays(want["out"]), "device vs reference")
+    assert (want["grads"] is not None) == bool(mo.num_arcs())
+    if mo.num_arcs():
+        gtn.backward(mo, seed_like(gtn, mo, rng))
+        for m, g in zip((ma, mb), want["grads"]):
+            assert np.array_equal(np.array(m.grad().weights_to_list(), np.float32).reshape(-1), np.array(g, np.float32))
 
 
 def test_list_overload_is_one_batched_call(gtn, on_device):

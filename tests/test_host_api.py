@@ -1,9 +1,10 @@
 """Host side of the gtn:: surface (SURVEY.md section 8(f) ranks 3-4): the rational operations, graph
 comparison, the two wire formats, Graphviz export and random sampling of gtn_b200.gtn against
 
-  * the UNMODIFIED reference compiled into oracle/_ref (same random graphs through both libraries;
-    outputs compared node by node and arc by arc, byte by byte for the wire formats), and
-  * hand-derived known answers that need no reference (they also run on a box without oracle/_ref).
+  * what the UNMODIFIED reference computed on the same seeded random graphs (tests/golden/reference_host.json,
+    made by tests/golden/make_golden.py; outputs compared node by node and arc by arc, byte by byte for the
+    wire formats), and
+  * hand-derived known answers.
 
 None of this touches the GPU: these functions are graph construction / tooling, exactly as in the
 reference (gtn/functions.cpp:93-223,253-318; gtn/utils.cpp; gtn/rand.cpp)."""
@@ -12,9 +13,7 @@ import os
 import numpy as np
 import pytest
 
-from oracle import pyoracle as po
-
-needs_ref = pytest.mark.skipif(not po.have_ref(), reason="oracle/_ref not built (needs /root/reference)")
+from tests import util
 
 
 @pytest.fixture(scope="module")
@@ -24,7 +23,7 @@ def gtn():
 
 
 # ---------------------------------------------------------------------------------------------
-# helpers: the same graph in both libraries
+# helpers
 
 
 def random_graph(rng, n_nodes, n_arcs, n_labels=3, p_eps=0.25, transducer=True, int_weights=True):
@@ -53,10 +52,6 @@ def ours_from(gtn, arrs, calc_grad=True):
     return g
 
 
-def ref_from(arrs, calc_grad=True):
-    return po.RefGraph.from_arrays(*arrs, calc_grad=calc_grad)
-
-
 def ours_arrays(g):
     n, a = g.num_nodes(), g.num_arcs()
     flags = np.array([(1 if g.is_start(i) else 0) | (2 if g.is_accept(i) else 0) for i in range(n)], np.uint8)
@@ -68,82 +63,81 @@ def ours_arrays(g):
                 w=np.array(g.weights_to_list(), np.float32).reshape(-1))
 
 
-def assert_same(ours, ref, what=""):
-    """Identical numbering: node flags and the arc list, in order."""
-    o, r = ours_arrays(ours), ref.arrays()
+def assert_same(ours, want, what=""):
+    """Identical numbering: node flags and the arc list, in order.  want: a graph of the golden fixture."""
+    o, r = ours_arrays(ours), util.graph_arrays(want)
     for k in ("flags", "src", "dst", "ilabel", "olabel", "w"):
         assert o[k].shape == r[k].shape, (what, k, o[k].shape, r[k].shape)
         assert np.array_equal(o[k], r[k]), (what, k, o[k], r[k])
 
 
 def seed_like(gtn, out_ours, rng):
-    """Random deltas for backward(g, grad): same arc count as the output, in both libraries."""
+    """Random deltas for backward(g, grad): same arc count as the output."""
     a = ours_arrays(out_ours)
     d = rng.integers(-5, 6, len(a["src"])).astype(np.float32)
-    arrs = (a["flags"], a["src"], a["dst"], a["ilabel"], a["olabel"], d)
-    return ours_from(gtn, arrs, calc_grad=False), ref_from(arrs, calc_grad=False)
+    return ours_from(gtn, (a["flags"], a["src"], a["dst"], a["ilabel"], a["olabel"], d), calc_grad=False)
+
+
+def golden(test, seed):
+    return util.golden_host()[test][str(seed)]
 
 
 # ---------------------------------------------------------------------------------------------
-# rational operations against the live reference
+# rational operations against the reference
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", range(6))
 def test_concat_closure_union_match_reference(gtn, seed):
     rng = np.random.default_rng(100 + seed)
     graphs = [random_graph(rng, int(rng.integers(1, 7)), int(rng.integers(0, 12))) for _ in range(4)]
     mine = [ours_from(gtn, g) for g in graphs]
-    theirs = [ref_from(g) for g in graphs]
+    want = iter(golden("concat", seed))
 
     for k in range(0, 5):
-        assert_same(gtn.concat(mine[:k]), po.ref_concat(theirs[:k]), "concat of %d" % k)
-        assert_same(gtn.union(mine[:k]), po.ref_union(theirs[:k]), "union of %d" % k)
-    assert_same(gtn.concat(mine[0], mine[1]), po.ref_concat(theirs[:2]), "binary concat")
-    for m, t in zip(mine, theirs):
-        assert_same(gtn.closure(m), po.ref_closure(t), "closure")
+        assert_same(gtn.concat(mine[:k]), next(want), "concat of %d" % k)
+        assert_same(gtn.union(mine[:k]), next(want), "union of %d" % k)
+    assert_same(gtn.concat(mine[0], mine[1]), next(want), "binary concat")
+    for m in mine:
+        assert_same(gtn.closure(m), next(want), "closure")
+        clones = [next(want) for _ in range(3)]
         for proj, name in ((0, gtn.Projection.NONE), (1, gtn.Projection.INPUT), (2, gtn.Projection.OUTPUT)):
-            assert_same(gtn.clone(m, name), po.ref_clone(t, proj), "clone %d" % proj)
-        assert_same(gtn.project_input(m), po.ref_clone(t, 1))
-        assert_same(gtn.project_output(m), po.ref_clone(t, 2))
+            assert_same(gtn.clone(m, name), clones[proj], "clone %d" % proj)
+        assert_same(gtn.project_input(m), clones[1])
+        assert_same(gtn.project_output(m), clones[2])
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", range(8))
 def test_remove_matches_reference(gtn, seed):
     rng = np.random.default_rng(200 + seed)
     arrs = random_graph(rng, int(rng.integers(2, 9)), int(rng.integers(1, 20)), p_eps=0.4)
-    m, t = ours_from(gtn, arrs), ref_from(arrs)
-    assert_same(gtn.remove(m), po.ref_remove(t), "remove epsilon")
-    assert_same(gtn.remove(m, 1), po.ref_remove(t, 1), "remove label 1")
-    assert_same(gtn.remove(m, -1, 1), po.ref_remove(t, -1, 1), "remove eps:1")
-    assert_same(gtn.remove(m, 0, 2), po.ref_remove(t, 0, 2), "remove 0:2")
+    m = ours_from(gtn, arrs)
+    want = golden("remove", seed)
+    assert_same(gtn.remove(m), want[0], "remove epsilon")
+    assert_same(gtn.remove(m, 1), want[1], "remove label 1")
+    assert_same(gtn.remove(m, -1, 1), want[2], "remove eps:1")
+    assert_same(gtn.remove(m, 0, 2), want[3], "remove 0:2")
     # list overload (bindings/python/gtn/_functions.cpp:195-203): labels broadcast
     for got in gtn.remove([m, m]):
-        assert_same(got, po.ref_remove(t), "remove list")
+        assert_same(got, want[0], "remove list")
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", range(4))
 def test_rational_gradients_match_reference(gtn, seed):
     """gradFuncs slice `deltas` by arc position (functions.cpp:98-110,158-163,193-202)."""
     rng = np.random.default_rng(300 + seed)
     graphs = [random_graph(rng, int(rng.integers(1, 6)), int(rng.integers(1, 9))) for _ in range(3)]
-    for op_ours, op_ref in ((gtn.concat, po.ref_concat), (gtn.union, po.ref_union),
-                            (lambda gs: gtn.closure(gs[0]), lambda gs: po.ref_closure(gs[0]))):
+    for op_ours, want in zip((gtn.concat, gtn.union, lambda gs: gtn.closure(gs[0])), golden("rational_grads", seed)):
         mine = [ours_from(gtn, g, calc_grad=(i != 1)) for i, g in enumerate(graphs)]
-        theirs = [ref_from(g, calc_grad=(i != 1)) for i, g in enumerate(graphs)]
-        out_m, out_t = op_ours(mine), op_ref(theirs)
-        seed_m, seed_t = seed_like(gtn, out_m, rng)
-        gtn.backward(out_m, seed_m)
-        po.ref_backward_with(out_t, seed_t)
+        out_m = op_ours(mine)
+        gtn.backward(out_m, seed_like(gtn, out_m, rng))
         used = 1 if op_ours not in (gtn.concat, gtn.union) else len(mine)
+        assert len(want) == used
         for i in range(used):
             if i == 1 and used > 1:
                 assert not mine[i].is_grad_available()
                 continue
             assert np.array_equal(np.array(mine[i].grad().weights_to_list(), np.float32).reshape(-1),
-                                  theirs[i].grad().weights()), (i, op_ours)
+                                  np.array(want[i], np.float32)), (i, op_ours)
 
 
 def test_remove_has_no_gradient(gtn):
@@ -213,7 +207,6 @@ def test_remove_known_answer(gtn):
 # comparison
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", range(10))
 def test_equal_and_isomorphic_agree_with_reference(gtn, seed):
     rng = np.random.default_rng(400 + seed)
@@ -237,11 +230,13 @@ def test_equal_and_isomorphic_agree_with_reference(gtn, seed):
     f2 = flags.copy()
     f2[0] ^= 2
     variants.append((f2, src, dst, il, ol, w))
-    m0, t0 = ours_from(gtn, base), ref_from(base)
-    for k, v in enumerate(variants):
-        m, t = ours_from(gtn, v), ref_from(v)
-        assert gtn.equal(m0, m) == po.ref_equal(t0, t), ("equal", k)
-        assert gtn.isomorphic(m0, m) == po.ref_isomorphic(t0, t), ("isomorphic", k)
+    m0 = ours_from(gtn, base)
+    want = golden("equal", seed)
+    assert len(want) == len(variants)
+    for k, (v, (equal, isomorphic)) in enumerate(zip(variants, want)):
+        m = ours_from(gtn, v)
+        assert gtn.equal(m0, m) == equal, ("equal", k)
+        assert gtn.isomorphic(m0, m) == isomorphic, ("isomorphic", k)
     assert gtn.equal(m0, ours_from(gtn, shuf)) and gtn.isomorphic(m0, ours_from(gtn, shuf))
 
 
@@ -277,34 +272,35 @@ def test_isomorphic_known_answers(gtn):
 # wire formats
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", range(5))
 def test_wire_formats_are_byte_compatible_with_reference(gtn, seed, tmp_path):
     rng = np.random.default_rng(500 + seed)
     n_arcs = int(rng.integers(0, 40))
     arrs = random_graph(rng, int(rng.integers(1, 30)), n_arcs, int_weights=(seed % 2 == 0))
-    m, t = ours_from(gtn, arrs), ref_from(arrs)
+    m = ours_from(gtn, arrs)
+    want = golden("wire", seed)
+    ref_bin, ref_txt = bytes.fromhex(want["bin"]), want["txt"].encode()
     # what we write is what the reference writes
-    assert gtn.dumpb(m) == po.ref_serialise(t, 0)
-    assert gtn.dumps(m).encode() == po.ref_serialise(t, 1)
-    assert repr(m).encode() == po.ref_serialise(t, 2)  # abbreviated above 20 nodes / arcs
+    assert gtn.dumpb(m) == ref_bin
+    assert gtn.dumps(m).encode() == ref_txt
+    assert repr(m) == want["repr"]  # abbreviated above 20 nodes / arcs
     dot = str(tmp_path / "g.dot")
     gtn.write_dot(m, dot)
-    assert open(dot, "rb").read() == po.ref_serialise(t, 3)
-    # what either writes, the other reads
-    assert_same(gtn.loadb(po.ref_serialise(t, 0)), t, "ours reads the reference's binary")
-    assert_same(m, po.ref_parse(gtn.dumpb(m), 0), "the reference reads our binary")
-    if arrs[0].any() and (arrs[0] & 2).any():  # the text format needs a start and an accept node
-        assert gtn.equal(gtn.loads(po.ref_serialise(t, 1).decode()), gtn.loads(gtn.dumps(m)))
-        back = po.ref_parse(gtn.dumps(m).encode(), 1)
-        assert_same(gtn.loads(gtn.dumps(m)), back, "text round trip through both parsers")
+    assert open(dot, "rb").read() == want["dot"].encode("utf-8")
+    # what either writes, the other reads (our bytes are the reference's, asserted above)
+    assert_same(gtn.loadb(ref_bin), want["graph"], "ours reads the reference's binary")
+    assert_same(m, want["from_bin"], "the reference reads our binary")
+    assert ("from_txt" in want) == bool(arrs[0].any() and (arrs[0] & 2).any())
+    if "from_txt" in want:  # the text format needs a start and an accept node
+        assert gtn.equal(gtn.loads(ref_txt.decode()), gtn.loads(gtn.dumps(m)))
+        assert_same(gtn.loads(gtn.dumps(m)), want["from_txt"], "text round trip through both parsers")
     # files
     fb, ft = str(tmp_path / "g.bin"), str(tmp_path / "g.txt")
     gtn.save(fb, m)
-    assert open(fb, "rb").read() == po.ref_serialise(t, 0)
+    assert open(fb, "rb").read() == ref_bin
     assert gtn.equal(gtn.load(fb), m)
     gtn.savetxt(ft, m)
-    assert open(ft, "rb").read() == po.ref_serialise(t, 1)
+    assert open(ft, "rb").read() == ref_txt
 
 
 def test_write_dot_with_symbols(gtn, tmp_path):
@@ -367,15 +363,13 @@ def acyclic(rng, n, extra):
             w.astype(np.float32))
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", range(6))
 def test_sample_draws_the_reference_path_under_the_same_srand(gtn, seed):
     """Both libraries draw from the C library's rand() in the same order (rand.cpp:14-47)."""
     rng = np.random.default_rng(600 + seed)
     arrs = random_graph(rng, 6, 14, p_eps=0.1) if seed % 2 else acyclic(rng, 7, 6)
-    m, t = ours_from(gtn, arrs), ref_from(arrs)
-    for s in range(5):
-        want = po.ref_sample(t, 1000 + s, 50)
+    m = ours_from(gtn, arrs)
+    for s, want in enumerate(golden("sample", seed)):
         gtn.srand(1000 + s)
         got = gtn.sample(m, 50)
         assert_same(got, want, "sample seed %d" % s)
@@ -416,7 +410,6 @@ def test_sample_properties_and_gradient(gtn):
 # operand is a gtn::linearGraph (tests/test_gpu_*.py)
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", range(24))
 def test_general_compose_matches_reference_structure_and_gradients(gtn, seed):
     rng = np.random.default_rng(700 + seed)
@@ -426,19 +419,16 @@ def test_general_compose_matches_reference_structure_and_gradients(gtn, seed):
     if intersect:  # acceptors
         a = (a[0], a[1], a[2], a[3], a[3].copy(), a[5])
         b = (b[0], b[1], b[2], b[3], b[3].copy(), b[5])
-    ma, mb, ta, tb = ours_from(gtn, a), ours_from(gtn, b), ref_from(a), ref_from(b)
+    ma, mb = ours_from(gtn, a), ours_from(gtn, b)
     if seed & 1:  # the three matchers: unsorted, singly sorted, doubly sorted (functions.cpp:225-251)
         ma.arc_sort(True)
-        ta.arc_sort(True)
     if seed & 2:
         mb.arc_sort(False)
-        tb.arc_sort(False)
     mo = gtn.intersect(ma, mb) if intersect else gtn.compose(ma, mb)
-    to = po.ref_op("intersect" if intersect else "compose", ta, tb)
-    assert_same(mo, to, "composed graph: same node and arc numbering as the reference")
+    want = golden("compose", seed)
+    assert_same(mo, want["out"], "composed graph: same node and arc numbering as the reference")
+    assert (want["grads"] is not None) == bool(mo.num_arcs())
     if mo.num_arcs():
-        seed_m, seed_t = seed_like(gtn, mo, rng)
-        gtn.backward(mo, seed_m)
-        po.ref_backward_with(to, seed_t)
-        for m, t in ((ma, ta), (mb, tb)):
-            assert np.array_equal(np.array(m.grad().weights_to_list(), np.float32).reshape(-1), t.grad().weights())
+        gtn.backward(mo, seed_like(gtn, mo, rng))
+        for m, g in zip((ma, mb), want["grads"]):
+            assert np.array_equal(np.array(m.grad().weights_to_list(), np.float32).reshape(-1), np.array(g, np.float32))

@@ -1,6 +1,6 @@
 """CPU tests: the C oracle against the committed golden vectors (made by the real
 reference, tests/golden/make_golden.py) and against the reference's own known-answer
-tests; plus, when oracle/_ref is present, against the live reference on random graphs."""
+tests; plus against the reference's results on seeded random graphs (tests/golden/reference_host.json)."""
 import numpy as np
 import pytest
 
@@ -113,60 +113,53 @@ def test_forward_known_answers():
     assert po.shortest_distance(g, True)[0] == 6.0
 
 
-@pytest.mark.skipif(not po.have_ref(), reason="oracle/_ref not built (needs /root/reference)")
+def rand_graph(rng, n, eps):
+    a = int(rng.integers(n, 3 * n))
+    flags = np.zeros(n, np.uint8)
+    flags[0] = 1
+    flags[-1] = 2
+    flags[int(rng.integers(0, n))] |= int(rng.integers(0, 4))
+    src = rng.integers(0, n, a).astype(np.int32)
+    dst = rng.integers(0, n, a).astype(np.int32)
+    il = rng.integers(-1 if eps else 0, 3, a).astype(np.int32)
+    ol = rng.integers(-1 if eps else 0, 3, a).astype(np.int32)
+    w = rng.uniform(-1, 1, a).astype(np.float32)
+    return flags, src, dst, il, ol, w
+
+
 @pytest.mark.parametrize("seed", range(4))
 def test_oracle_vs_live_reference_random(seed):
-    """Exact structural equality of compose (all three matchers), scores, gradients, paths."""
+    """Exact structural equality of compose (all three matchers), scores, gradients, paths, against what the
+    reference computed on the same seeded graphs (tests/golden/reference_host.json)."""
+    gold = util.golden_host()["oracle"][str(seed)]
+    want = iter(gold["compose"])
     rng = np.random.default_rng(100 + seed)
     for _ in range(10):
         n1, n2 = int(rng.integers(2, 8)), int(rng.integers(2, 8))
-
-        def rand_graph(n, eps):
-            a = int(rng.integers(n, 3 * n))
-            flags = np.zeros(n, np.uint8)
-            flags[0] = 1
-            flags[-1] = 2
-            flags[int(rng.integers(0, n))] |= int(rng.integers(0, 4))
-            src = rng.integers(0, n, a).astype(np.int32)
-            dst = rng.integers(0, n, a).astype(np.int32)
-            il = rng.integers(-1 if eps else 0, 3, a).astype(np.int32)
-            ol = rng.integers(-1 if eps else 0, 3, a).astype(np.int32)
-            w = rng.uniform(-1, 1, a).astype(np.float32)
-            return flags, src, dst, il, ol, w
-
         eps = bool(rng.integers(0, 2))
-        a1, a2 = rand_graph(n1, eps), rand_graph(n2, eps)
+        a1, a2 = rand_graph(rng, n1, eps), rand_graph(rng, n2, eps)
         g1, g2 = po.Graph.from_arrays(*a1), po.Graph.from_arrays(*a2)
-        r1, r2 = po.RefGraph.from_arrays(*a1), po.RefGraph.from_arrays(*a2)
         sort_mode = int(rng.integers(0, 4))
         if sort_mode & 1:
             g1.arc_sort(True)
-            r1.arc_sort(True)
         if sort_mode & 2:
             g2.arc_sort(False)
-            r2.arc_sort(False)
-        for mode, name in ((0, "compose"), (1, "intersect")):
+        for mode in (0, 1):
             mine = po.compose(g1, g2) if mode == 0 else po.intersect(g1, g2)
-            ref = po.ref_op(name, r1, r2)
-            ma, ra = mine.arrays(), ref.arrays()
-            assert mine.num_nodes == ref.num_nodes and mine.num_arcs == ref.num_arcs
+            ma, ra = mine.arrays(), util.graph_arrays(next(want))
+            assert mine.num_nodes == len(ra["flags"]) and mine.num_arcs == len(ra["src"])
             for k in ("flags", "src", "dst", "ilabel", "olabel", "w"):
                 assert np.array_equal(ma[k], ra[k]), k
     # DAGs: scores, gradients, best paths
-    for _ in range(10):
+    for dag in gold["dags"]:
         n = int(rng.integers(2, 30))
         arrs = util.random_dag(rng, n, int(rng.integers(n, 4 * n)), int_weights=bool(rng.integers(0, 2)))
         g = po.Graph.from_arrays(*arrs)
-        r = po.RefGraph.from_arrays(*arrs)
-        for tropical, name in ((False, "forward_score"), (True, "viterbi_score")):
+        for k, tropical in enumerate((False, True)):
             s, gr = po.forward_score_and_grad(g, tropical)
-            rs = po.ref_op(name, r)
-            assert util.close(s, rs.item(), rtol=1e-6)
-            po.ref_backward(rs)
-            rg = r.grad().weights()
+            assert util.close(s, dag["scores"][k], rtol=1e-6)
+            rg = np.array(dag["grads"][k], np.float32)
             assert np.abs(rg - gr).max() < 1e-6
-            po.libref().ref_graph_zero_grad(r.h)
         path = po.shortest_path(g)
-        rp = po.ref_op("viterbi_path", r).arrays()
-        assert np.array_equal(g.arrays()["ilabel"][path], rp["ilabel"])
-        assert np.array_equal(g.arrays()["w"][path], rp["w"])
+        assert np.array_equal(g.arrays()["ilabel"][path], np.array(dag["path_ilabel"], np.int32))
+        assert np.array_equal(g.arrays()["w"][path], np.array(dag["path_w"], np.float32))

@@ -1,7 +1,32 @@
-"""Helpers shared by the tests: graph builders and tolerances."""
+"""Helpers shared by the tests: graph builders, tolerances and the golden fixtures."""
+import functools
+import json
+import os
+
 import numpy as np
 
 from gtn_b200 import capi
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+GRAPH_KEYS = ("flags", "src", "dst", "ilabel", "olabel", "w")
+
+
+@functools.lru_cache(maxsize=None)
+def golden_host():
+    """tests/golden/reference_host.json: the reference's outputs for the seeded host-side graph tests."""
+    with open(os.path.join(GOLDEN, "reference_host.json")) as f:
+        return json.load(f)
+
+
+def golden_configs():
+    """tests/golden/reference_configs.npz: the reference's outputs at the BASELINE.json configurations."""
+    return np.load(os.path.join(GOLDEN, "reference_configs.npz"))
+
+
+def graph_arrays(rec):
+    """A graph stored in a golden fixture, [flags, src, dst, ilabel, olabel, w] -> dict of arrays."""
+    return {k: np.array(v, np.float32 if k == "w" else (np.uint8 if k == "flags" else np.int32))
+            for k, v in zip(GRAPH_KEYS, rec)}
 
 # north_star tolerance: 1e-4 relative for scores and gradients; the small
 # absolute term is the one the reference's own tests use (criterion_test.cpp:127)
