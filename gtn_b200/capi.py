@@ -91,6 +91,9 @@ SYMBOLS = [
     ("gtnb_ctc_loss", C.c_int,
      [_vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _i32p, _i32p, _i32p, C.c_int, _f32p, _vp,
       C.c_int]),
+    ("gtnb_ctc_align", C.c_int,
+     [_vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _i32p, _i32p, _i32p, C.c_int, C.c_int, _vp, _vp, C.c_int,
+      _f32p]),
 ]
 
 _lib = None
@@ -358,6 +361,52 @@ class Ctx:
             e_dev.free()
             g_dev.free()
         return losses, grads
+
+    @staticmethod
+    def _align_args(emissions, targets, input_lens):
+        e = np.ascontiguousarray(emissions, dtype=np.float32)
+        lens = np.asarray([len(t) for t in targets], np.int32)
+        cat = np.ascontiguousarray(
+            np.concatenate([np.asarray(t, np.int32) for t in targets]) if len(targets) else np.zeros(0, np.int32),
+            np.int32)
+        il = None if input_lens is None else np.ascontiguousarray(input_lens, np.int32)
+        return e, lens, cat, il
+
+    def ctc_align(self, emissions, targets, blank=0, input_lens=None, arc_sorted=True, want_states=False):
+        """Host-buffer entry of gtnb_ctc_align: emissions [B,T,C] -> (labels [B,T], scores [B], states [B,T] or
+        None): the best path of intersect(ctcGraph(target_b), emissions_b), -1 past input_lens[b] or without a path."""
+        e, lens, cat, il = self._align_args(emissions, targets, input_lens)
+        B, T, Cn = e.shape
+        labels = np.full((B, max(T, 1)), -7, np.int32)
+        states = np.full_like(labels, -7) if want_states else None
+        scores = np.zeros(max(B, 1), np.float32)
+        self._check(lib().gtnb_ctc_align(
+            self.h, B, T, Cn, e.ctypes.data, 0, _p(il, _i32p), _p(cat, _i32p), _p(lens, _i32p), int(blank),
+            int(arc_sorted), labels.ctypes.data, None if states is None else states.ctypes.data, 0,
+            _p(scores, _f32p)))
+        return labels[:, :T], scores[:B], None if states is None else states[:, :T]
+
+    def ctc_align_dev(self, emissions, targets, blank=0, input_lens=None, arc_sorted=True, want_states=False):
+        """Device-buffer entry of gtnb_ctc_align: emissions uploaded once, labels / states written to device
+        buffers and downloaded afterwards -> the same as ctc_align."""
+        e, lens, cat, il = self._align_args(emissions, targets, input_lens)
+        B, T, Cn = e.shape
+        scores = np.zeros(max(B, 1), np.float32)
+        e_dev = self.to_device(e)
+        l_dev = self.alloc(4 * max(B * T, 1))
+        s_dev = self.alloc(4 * max(B * T, 1)) if want_states else None
+        try:
+            self._check(lib().gtnb_ctc_align(
+                self.h, B, T, Cn, e_dev.ptr, 1, _p(il, _i32p), _p(cat, _i32p), _p(lens, _i32p), int(blank),
+                int(arc_sorted), l_dev.ptr, None if s_dev is None else s_dev.ptr, 1, _p(scores, _f32p)))
+            labels = l_dev.download((B, T), np.int32)
+            states = None if s_dev is None else s_dev.download((B, T), np.int32)
+        finally:
+            e_dev.free()
+            l_dev.free()
+            if s_dev is not None:
+                s_dev.free()
+        return labels, scores[:B], states
 
 
 class Lattice:

@@ -470,6 +470,231 @@ extern "C" int gtnb_viterbi_dense(
 }
 
 /*
+ * CTC forced alignment for a whole minibatch: viterbiPath + viterbiScore of intersect(ctcGraph(target_b), e_b)
+ * on the implicit lattice (k_align.cu).  Utterances outside the kernel's envelope are rerun one by one on the
+ * lattice route (compose + k_order.cu + the MODE_PATH kernels), which reproduces the reference's handling of
+ * non-finite weights and unmatched labels arc by arc.
+ */
+namespace {
+
+/* the CTC graph of benchmarks/ctc.cpp:40-58 as a host view, out lists in arcSort order when `sorted` */
+struct CtcView {
+  std::vector<uint8_t> flags;
+  std::vector<int32_t> src, dst, lab, out_ptr, out_arcs;
+  gtnb_graph_view v;
+  CtcView(const int32_t* y, int U, int blank, bool sorted) {
+    const int L = 2 * U + 1;
+    flags.assign(L, 0);
+    flags[0] |= 1;
+    flags[L - 1] |= 2;
+    if (L >= 2) flags[L - 2] |= 2;
+    auto add = [&](int s, int d, int l) {
+      src.push_back(s);
+      dst.push_back(d);
+      lab.push_back(l);
+    };
+    for (int l = 0; l < L; l++) {
+      const int label = (l & 1) ? y[(l - 1) / 2] : blank;
+      add(l, l, label);
+      if (l > 0) add(l - 1, l, label);
+      if ((l & 1) && l > 1 && label != y[(l - 3) / 2]) add(l - 2, l, label);
+    }
+    out_ptr.assign(L + 1, 0);
+    for (int s : src) out_ptr[s + 1]++;
+    for (int n = 0; n < L; n++) out_ptr[n + 1] += out_ptr[n];
+    out_arcs.resize(src.size());
+    std::vector<int32_t> pos(out_ptr.begin(), out_ptr.end() - 1);
+    for (size_t a = 0; a < src.size(); a++) out_arcs[pos[src[a]]++] = (int32_t)a;
+    if (sorted) // Graph::arcSort (graph.cpp:162-177): stable on these lists of <= 3 arcs
+      for (int n = 0; n < L; n++)
+        std::stable_sort(out_arcs.begin() + out_ptr[n], out_arcs.begin() + out_ptr[n + 1],
+                         [&](int a, int b) { return lab[a] < lab[b]; });
+    std::memset(&v, 0, sizeof(v));
+    v.num_nodes = L;
+    v.num_arcs = (int32_t)src.size();
+    v.node_flags = flags.data();
+    v.arc_src = src.data();
+    v.arc_dst = dst.data();
+    v.arc_ilabel = v.arc_olabel = lab.data();
+    v.out_ptr = out_ptr.data();
+    v.out_arcs = out_arcs.data();
+  }
+};
+
+/* utterance b on the lattice route: labels / states rows [T] (states nullable) and the score, on the host */
+int ctc_align_lattice(gtnb_ctx* ctx, const CtcView& g, int Tb, int T, int C, const float* e_dev, int32_t* labels,
+                      int32_t* states, float* score) {
+  const bool ties = ctx->exact_ties;
+  ctx->exact_ties = true;
+  gtnb_lattice* lat = nullptr;
+  int rc = gtnb_compose_linear(ctx, 1, &g.v, 1, 0, &Tb, C, e_dev, (int64_t)Tb * C, &lat);
+  ctx->exact_ties = ties;
+  if (rc) return rc;
+  std::vector<int32_t> arcs(std::max(Tb, 1), -1), il(std::max(Tb, 1), -1);
+  int32_t len = -1;
+  rc = gtnb_viterbi_path(ctx, lat, Tb, arcs.data(), il.data(), nullptr, nullptr, &len, nullptr);
+  if (!rc) rc = gtnb_forward(ctx, lat, 1, score, nullptr);
+  std::vector<int32_t> gi;
+  if (!rc && states && len > 0) {
+    int32_t nn = 0, na = 0;
+    rc = gtnb_lattice_sizes(ctx, lat, &nn, &na);
+    gi.resize(std::max(na, 1));
+    if (!rc) rc = gtnb_lattice_download(ctx, lat, 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, gi.data(), nullptr);
+  }
+  gtnb_lattice_destroy(ctx, lat);
+  if (rc) return rc;
+  for (int t = 0; t < T; t++) {
+    const bool on = t < len;
+    labels[t] = on ? il[t] : -1;
+    if (states) states[t] = on ? g.dst[gi[arcs[t]]] : -1;
+  }
+  return GTNB_OK;
+}
+
+} // namespace
+
+static int ctc_align_run(
+    gtnb_ctx* ctx, int B, int T, int C, const float* emissions, int emissions_on_device, const int32_t* input_lens,
+    const int32_t* targets, const int32_t* target_lens, int blank, int arc_sorted, int32_t* labels, int32_t* states,
+    int outputs_on_device, float* scores_host, std::vector<int32_t>& status) {
+  if (!ctx || B < 0 || T < 0 || C <= 0 || (B > 0 && (!target_lens || !scores_host)) ||
+      ((long long)B * T > 0 && (!emissions || !labels)))
+    return fail(ctx, GTNB_ERR_INVALID_ARGUMENT, "gtnb_ctc_align: bad arguments");
+  std::vector<int32_t> small(3ll * B);
+  long long tot_t = 0;
+  int maxL = 1;
+  for (int b = 0; b < B; b++) {
+    const int U = target_lens[b];
+    if (U < 0) return fail(ctx, GTNB_ERR_INVALID_ARGUMENT, "gtnb_ctc_align: negative target length");
+    if (U > 0 && !targets) return fail(ctx, GTNB_ERR_INVALID_ARGUMENT, "gtnb_ctc_align: targets is NULL");
+    const int Tb = input_lens ? input_lens[b] : T;
+    if (Tb < 0 || Tb > T) return fail(ctx, GTNB_ERR_INVALID_ARGUMENT, "gtnb_ctc_align: input_lens out of range");
+    const int32_t* y = targets + tot_t;
+    int out_deg = U > 0 ? 2 : 1;
+    for (int u = 1; u < U; u++)
+      if (y[u] != y[u - 1]) out_deg = 3; // a skip arc
+    if (arc_sorted && out_deg > C)
+      return fail(ctx, GTNB_ERR_UNSUPPORTED,
+                  "gtnb_ctc_align: sorted CTC graph with out-degree > C (the reference's doubly-sorted matcher then "
+                  "enumerates arcs in emission-label order, which neither route reproduces)");
+    small[b] = Tb;
+    small[B + b] = (int32_t)tot_t;
+    small[2 * B + b] = U;
+    maxL = std::max(maxL, 2 * U + 1);
+    tot_t += U;
+  }
+  if (B == 0) return GTNB_OK;
+  GTNB_CUDA(ctx, cudaSetDevice(ctx->device));
+  const long long per = (long long)T * C;
+  const long long n_out = (long long)B * T;
+  int rc = GTNB_OK;
+  float* e_dev = nullptr;
+  int32_t *small_dev = nullptr, *lab_dev = nullptr, *st_dev = nullptr;
+  uint8_t* bp = nullptr;
+  float* res_dev = nullptr; // [scores | status]
+#define TRY(x)                 \
+  do {                         \
+    if ((rc = (x))) goto done; \
+  } while (0)
+#define TRYCUDA(call)                                      \
+  do {                                                     \
+    cudaError_t e__ = (call);                              \
+    if (e__ != cudaSuccess) {                              \
+      rc = cuda_fail(ctx, e__, #call, __FILE__, __LINE__); \
+      goto done;                                           \
+    }                                                      \
+  } while (0)
+  if (emissions_on_device) {
+    e_dev = const_cast<float*>(emissions);
+  } else {
+    TRY(dev_alloc(ctx, &e_dev, per * B));
+    if (per) TRYCUDA(cudaMemcpyAsync(e_dev, emissions, sizeof(float) * per * B, cudaMemcpyHostToDevice, ctx->stream));
+  }
+  if (outputs_on_device) {
+    lab_dev = labels;
+    st_dev = states;
+  } else {
+    TRY(dev_alloc(ctx, &lab_dev, n_out));
+    if (states) TRY(dev_alloc(ctx, &st_dev, n_out));
+  }
+  TRY(dev_alloc(ctx, &small_dev, 3ll * B + tot_t));
+  TRY(dev_alloc(ctx, &bp, (long long)B * T * (long long)ctc_align_bp_pitch(maxL)));
+  TRY(dev_alloc(ctx, &res_dev, 2ll * B));
+  TRY(stage_begin(ctx));
+  TRY(stage_upload(ctx, small_dev, small.data(), sizeof(int32_t) * small.size()));
+  if (tot_t) TRY(stage_upload(ctx, small_dev + 3ll * B, targets, sizeof(int32_t) * tot_t));
+  TRY(stage_end(ctx));
+  TRY(launch_ctc_align(ctx, B, T, C, blank, arc_sorted, maxL, small_dev, e_dev, per, bp, lab_dev, st_dev, res_dev,
+                       reinterpret_cast<int32_t*>(res_dev + B)));
+  if (!outputs_on_device && n_out) {
+    TRYCUDA(cudaMemcpyAsync(labels, lab_dev, sizeof(int32_t) * n_out, cudaMemcpyDeviceToHost, ctx->stream));
+    if (states)
+      TRYCUDA(cudaMemcpyAsync(states, st_dev, sizeof(int32_t) * n_out, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  TRY(readback_reserve(ctx, 2 * sizeof(float) * B));
+  TRYCUDA(cudaMemcpyAsync(ctx->readback, res_dev, 2 * sizeof(float) * B, cudaMemcpyDeviceToHost, ctx->stream));
+  TRYCUDA(cudaStreamSynchronize(ctx->stream));
+  std::memcpy(scores_host, ctx->readback, sizeof(float) * B);
+  status.assign(reinterpret_cast<int32_t*>(ctx->readback) + B, reinterpret_cast<int32_t*>(ctx->readback) + 2 * B);
+done:
+  if (!emissions_on_device) dev_free(ctx, e_dev);
+  if (!outputs_on_device) {
+    dev_free(ctx, lab_dev);
+    dev_free(ctx, st_dev);
+  }
+  dev_free(ctx, small_dev);
+  dev_free(ctx, bp);
+  dev_free(ctx, res_dev);
+  return rc;
+#undef TRY
+#undef TRYCUDA
+}
+
+extern "C" int gtnb_ctc_align(
+    gtnb_ctx* ctx, int B, int T, int C, const float* emissions, int emissions_on_device, const int32_t* input_lens,
+    const int32_t* targets, const int32_t* target_lens, int blank, int arc_sorted, int32_t* labels, int32_t* states,
+    int outputs_on_device, float* scores_host) {
+  std::vector<int32_t> status;
+  if (ctx) arena_begin(ctx);
+  int rc = ctc_align_run(ctx, B, T, C, emissions, emissions_on_device, input_lens, targets, target_lens, blank,
+                         arc_sorted, labels, states, outputs_on_device, scores_host, status);
+  if (ctx) arena_end(ctx);
+  // the utterances outside the kernel's envelope, on the lattice route (outside the call's arena: their lattices
+  // are large and rare, the arena keeps the size of the last call)
+  long long off = 0;
+  bool rerun = false;
+  for (int b = 0; b < B && rc == GTNB_OK; off += target_lens[b], b++) {
+    if (!status[b]) continue;
+    rerun = true;
+    const int Tb = input_lens ? input_lens[b] : T;
+    const CtcView g(targets + off, target_lens[b], blank, arc_sorted != 0);
+    std::vector<int32_t> lab_row(std::max(T, 1)), st_row(std::max(T, 1));
+    float* e_b = nullptr;
+    if (emissions_on_device) {
+      e_b = const_cast<float*>(emissions) + (long long)b * T * C;
+    } else if ((rc = dev_alloc(ctx, &e_b, (long long)Tb * C)) == GTNB_OK && Tb) {
+      const cudaError_t ce = cudaMemcpyAsync(e_b, emissions + (long long)b * T * C, sizeof(float) * Tb * C,
+                                             cudaMemcpyHostToDevice, ctx->stream);
+      if (ce != cudaSuccess) rc = cuda_fail(ctx, ce, "cudaMemcpyAsync", __FILE__, __LINE__);
+    }
+    if (rc == GTNB_OK)
+      rc = ctc_align_lattice(ctx, g, Tb, T, C, e_b, lab_row.data(), states ? st_row.data() : nullptr, &scores_host[b]);
+    if (!emissions_on_device) dev_free(ctx, e_b);
+    if (rc || !T) continue;
+    const size_t row = sizeof(int32_t) * T;
+    if (outputs_on_device) {
+      rc = gtnb_memcpy_h2d(ctx, labels + (long long)b * T, lab_row.data(), row);
+      if (!rc && states) rc = gtnb_memcpy_h2d(ctx, states + (long long)b * T, st_row.data(), row);
+    } else {
+      std::memcpy(labels + (long long)b * T, lab_row.data(), row);
+      if (states) std::memcpy(states + (long long)b * T, st_row.data(), row);
+    }
+  }
+  if (rc == GTNB_OK && outputs_on_device && rerun) rc = gtnb_ctx_synchronize(ctx);
+  return rc;
+}
+
+/*
  * ASG criterion for a whole minibatch (test/criterion_test.cpp:244-305, examples/asg.cpp:59-81):
  *   loss_b = forwardScore(compose(e_b, transitions))
  *          - forwardScore(compose(compose(fal_b, transitions), e_b))

@@ -336,6 +336,13 @@ int ensure_side_streams(gtnb_ctx* ctx, int n_streams, int n_events);
 int launch_viterbi_dense(
     gtnb_ctx* ctx, int B, int T_max, int C, const int32_t* T_dev, const float* emis, int64_t stride,
     const float* trans_dev, uint8_t* bp, int32_t* paths, float* scores);
+// kernels (k_align.cu): CTC forced alignment on the implicit lattice; small_dev = [T_b | target offsets | U | targets],
+// outputs [B][T_max]; status[b] != 0: utterance b is outside the kernel's envelope and was not written
+int launch_ctc_align(
+    gtnb_ctx* ctx, int B, int T_max, int C, int blank, int arc_sorted, int maxL, const int32_t* small_dev,
+    const float* emis, int64_t stride, uint8_t* bp, int32_t* labels, int32_t* states, float* scores,
+    int32_t* status);
+size_t ctc_align_bp_pitch(int maxL); // bytes of one back-pointer row
 // kernels (k_compose.cu)
 int launch_compose(gtnb_ctx* ctx, gtnb_lattice* lat, cudaEvent_t emissions_ready = nullptr);
 int launch_compose_grad(gtnb_ctx* ctx, gtnb_lattice* lat, float* grad_graph, float* grad_emis, int64_t grad_stride);

@@ -121,3 +121,37 @@ class ASGLossFunction(torch.autograd.Function):
 
 def asg_loss(emissions, transitions, targets, reduction="mean", allreduce=True):
     return ASGLossFunction.apply(emissions, transitions, targets, reduction, allreduce)
+
+
+@torch.no_grad()
+def ctc_align(emissions, targets, input_lengths=None, blank=0, arc_sorted=True):
+    """CTC forced alignment: the best path of intersect(ctcGraph(target_b), emissions_b) (gtnb_ctc_align).
+
+    emissions: float32 CUDA tensor [B, T, C]; targets: list of 1-D int sequences; input_lengths: per-utterance
+    frame counts (sequence or tensor), default T.  Returns (labels int32 [B, T], states int32 [B, T],
+    scores float32 [B]) on the emissions' device: the path's label and CTC graph node per frame (-1 past
+    input_lengths[b] or when no path exists) and its viterbiScore (-inf without a path).  Runs on the current
+    stream; no autograd.
+    """
+    assert emissions.is_cuda and emissions.dtype == torch.float32 and emissions.dim() == 3
+    e = emissions.detach().contiguous()
+    B, T, Cn = e.shape
+    stream = torch.cuda.current_stream(e.device).cuda_stream
+    g = _ctx_for(e.device, stream)
+    lens = np.asarray([len(t) for t in targets], np.int32)
+    cat = np.ascontiguousarray(
+        np.concatenate([np.asarray(t, np.int32) for t in targets]) if B else np.zeros(0, np.int32), np.int32)
+    il = None
+    if input_lengths is not None:
+        if torch.is_tensor(input_lengths):
+            input_lengths = input_lengths.detach().cpu().numpy()
+        il = np.ascontiguousarray(input_lengths, np.int32)
+        assert il.shape == (B,)
+    labels = torch.empty((B, T), dtype=torch.int32, device=e.device)
+    states = torch.empty((B, T), dtype=torch.int32, device=e.device)
+    scores = np.zeros(max(B, 1), np.float32)
+    g._check(capi.lib().gtnb_ctc_align(
+        g.h, B, T, Cn, e.data_ptr(), 1, None if il is None else il.ctypes.data_as(capi._i32p),
+        cat.ctypes.data_as(capi._i32p), lens.ctypes.data_as(capi._i32p), int(blank), int(arc_sorted),
+        labels.data_ptr(), states.data_ptr(), 1, scores.ctypes.data_as(capi._f32p)))
+    return labels, states, torch.from_numpy(scores[:B]).to(e.device)

@@ -387,6 +387,40 @@ int gtnb_viterbi_dense(
     int32_t* paths_host,
     float* scores_host);
 
+/*
+ * CTC forced alignment for a whole minibatch: for utterance b, with T_b = input_lens ? input_lens[b] : T,
+ *   labels[b][t] (t < T_b) = ilabel of the t-th arc of viterbiPath(intersect(ctc_b, linearGraph(T_b, C; e_b)))
+ *   scores_host[b]         = viterbiScore of the same lattice (shortest.cpp:190-272)
+ * ctc_b is the CTC graph of benchmarks/ctc.cpp:40-58 for target b with `blank`, after arcSort() when
+ * arc_sorted != 0 (as benchmarks/ctc.cpp:56 and the criterion do), in insertion order otherwise; the two differ
+ * only in how exact score ties are broken.  Paths and scores are bit-identical to the reference's, ties
+ * included.  states (nullable) [B][T]: the CTC graph node (0 .. 2U_b) the path is in after frame t.
+ * Where there is no accepting path, or at t >= T_b, labels / states are -1; with no accepting path the score
+ * is -inf (T_b = 0: 0 when U_b = 0).  emissions [B][T][C] (device pointer when emissions_on_device);
+ * labels / states are device pointers when outputs_on_device, else host.  Targets, target_lens, input_lens
+ * are host arrays as for gtnb_ctc_loss.
+ * The lattice is never built (k_align.cu); utterances with a non-finite emission on a lattice arc, labels or
+ * blank outside [0, C), or more than 2047 target labels are computed on the lattice route instead.
+ * GTNB_ERR_UNSUPPORTED when arc_sorted and a CTC graph node has more out-arcs than C (C < 3): the reference's
+ * doubly-sorted matcher then orders a state's arcs by emission label, which neither route reproduces.
+ */
+int gtnb_ctc_align(
+    gtnb_ctx* ctx,
+    int B,
+    int T,
+    int C,
+    const float* emissions,
+    int emissions_on_device,
+    const int32_t* input_lens,
+    const int32_t* targets,
+    const int32_t* target_lens,
+    int blank,
+    int arc_sorted,
+    int32_t* labels,
+    int32_t* states,
+    int outputs_on_device,
+    float* scores_host);
+
 #ifdef __cplusplus
 }
 #endif
